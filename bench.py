@@ -4,7 +4,7 @@ synthetic 24 kHz audio per GPU (125 frames of 80 ms each, one frame of every str
 sequence), seeded synthetic weights.  Metric: codec frames/s (one frame = 1920 samples encoded to
 8 tokens and decoded back); real-time streams = frames/s / 12.5.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" = one pass over the whole batch: 125 streaming frames x 256 streams (encode + decode).
 `value` is measured with the 10 s inputs already resident in HBM; `e2e` copies every 80 ms chunk
@@ -42,6 +42,7 @@ STREAMS, SECONDS = 256, 10
 FRAMES = int(SECONDS * 12.5)
 FRAME = 1920
 METRIC, UNIT = "codec_frames_per_s", "frames/s"
+DUMP_WAV_STREAMS = 32     # --dump-outputs: 32 x 10 s of float32 audio = 31 MB
 WORKLOAD = f"mimi_streaming_encode_decode_B{STREAMS}x{SECONDS}s_24kHz"
 
 
@@ -196,7 +197,15 @@ def run_ours(args):
 
     state = {"entered": False}
 
-    def step(resident: bool, cold: bool = True):
+    # --dump-outputs: the last timed step's tokens (every stream) and waveforms (a fixed seeded sample of streams) are
+    # copied into these preallocated buffers as they are produced, so the timed loop allocates nothing extra
+    record = None
+    if args.dump_outputs and rank == 0:
+        rows = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:DUMP_WAV_STREAMS].sort().values.to(dev)
+        record = {"rows": rows, "codes": torch.empty(FRAMES, B, 8, 1, dtype=torch.int64, device=dev),
+                  "wav": torch.empty(FRAMES, rows.numel(), 1, FRAME, device=dev)}
+
+    def step(resident: bool, cold: bool = True, rec=None):
         """125 streaming frames for all streams: encode chunk -> decode tokens.  One streaming scope is
         kept for the whole run (buffers + CUDA graphs are reused) and reset between passes (cold = every pass starts
         like a new 10 s stream; cold False keeps the state: the transformer rings stay full)."""
@@ -213,6 +222,9 @@ def run_ours(args):
             if not resident:
                 out_codes_host.copy_(codes, non_blocking=True)
                 out_wav_host.copy_(wav, non_blocking=True)
+            if rec is not None:
+                rec["codes"][i].copy_(codes)
+                torch.index_select(wav, 0, rec["rows"], out=rec["wav"][i])
         if not resident:
             torch.cuda.current_stream().synchronize()
 
@@ -221,13 +233,13 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(resident: bool, steps: int, cold: bool = True):
+    def timed(resident: bool, steps: int, cold: bool = True, rec=None):
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         l0 = _lib.launch_count()
         e0.record()
-        for _ in range(steps):
-            step(resident, cold)
+        for s in range(steps):
+            step(resident, cold, rec if s == steps - 1 else None)
         e1.record()
         barrier()
         ms, _ = reduce_timing(e0.elapsed_time(e1), B * FRAMES * steps, device=dev)  # max over ranks
@@ -247,8 +259,11 @@ def run_ours(args):
     for _ in range(max(3, args.warmup)):
         step(True)
     with ClockSampler(local) as cs:
-        ms, _ = timed(True, args.steps)
+        ms, _ = timed(True, args.steps, rec=record)
     clocks = cs.summary()
+    if record is not None:
+        dump_outputs(args.dump_outputs, record)
+        record = None
     for _ in range(1):
         step(False)
     ms_e2e, _ = timed(False, args.steps)
@@ -322,6 +337,19 @@ def run_ours(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, record):
+    """What the headline's last timed step returned to its caller, as float32 .npy files:
+    codes.npy [streams, 8, frames] (token ids, exact in float32) and wav.npy [DUMP_WAV_STREAMS, 1, frames * 1920]
+    (the decoded waveform of the streams listed in wav_rows.npy, a fixed seeded sample of the batch)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"codes": record["codes"][..., 0].permute(1, 2, 0),
+              "wav": record["wav"].permute(1, 2, 0, 3).reshape(record["wav"].shape[1], 1, -1),
+              "wav_rows": record["rows"]}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.float().cpu().numpy())
 
 
 def roofline_pass(m, x_dev, B, dev):
@@ -708,7 +736,14 @@ def main():
     ap.add_argument("--no-lm", dest="no_lm", action="store_true", help="skip the secondary LM decode-step measurement")
     ap.add_argument("--frames", type=int, default=FRAMES,
                     help="frames per stream per step (profiling aid: ncu runs use a short pass; the default 125 is the bench)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last timed step's outputs (rank 0's streams) to DIR/*.npy "
+                         "so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU arm (--impl ours)")
     if args.frames != FRAMES:
         FRAMES = args.frames
         WORKLOAD += f"_SHORT{FRAMES}frames"

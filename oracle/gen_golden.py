@@ -27,6 +27,9 @@ from . import mimi_oracle as O
 from . import mimi_spec as S
 
 GOLDEN = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+# intra-op threads of every fixture run: torch's CPU float32 convolutions split their sums by thread count, so the
+# tests that compare the oracle with the fixtures bit for bit (or to 1e-6) use the same count
+GOLDEN_THREADS = 8
 
 
 def weights_digest(w) -> str:
@@ -75,7 +78,7 @@ def build_reference_mimimodel(w):
 
 
 def main():
-    torch.set_num_threads(min(8, os.cpu_count() or 1))
+    torch.set_num_threads(GOLDEN_THREADS)
     os.makedirs(GOLDEN, exist_ok=True)
     cfg = S.OFFICIAL
     w = S.synthetic_weights(cfg, seed=41, codebook_scale=S.CODEBOOK_SCALE)

@@ -1,29 +1,51 @@
-"""Generate tests/golden/lm_small.npz by running the UNMODIFIED reference GPT (streaming decode) here.
+"""Generate tests/golden/lm_small.npz and lm_round2.npz by running the UNMODIFIED reference GPT (streaming decode).
 
-Run:  python -m oracle.gen_golden_lm      (needs /root/reference)
+Run:  python -m oracle.gen_golden_lm <MLLM_v2 directory of the original RSTnet checkout>
 
 The reference `models.llama_streaming.GPT` (small config, seeded synthetic weights from
 oracle/lm_oracle.synthetic_weights) is stepped for a few frames under `with gpt.streaming(B)` with
 greedy sampling, in fp32 and in bf16; the oracle restatement must reproduce it bit for bit, and the
 reference outputs are stored.
+
+Every fixture stays under 1 MB, so the large tensors are stored in a smaller but equivalent form:
+  *_sha256      SHA-256 of the float32 bytes, for tensors the tests compare bit for bit;
+  *_bits        bf16 results as their raw 16-bit patterns (lossless);
+  *_sampled     a fixed seeded sample of vocabulary columns (*_cols), for tensors compared within a tolerance;
+  lora_update_* the reference's merged weight minus the seeded base weight, as rank-r factors u @ v (exact to 1e-7).
 """
 from __future__ import annotations
 
+import hashlib
 import os
 import sys
 
 os.environ.setdefault("NO_TORCH_COMPILE", "1")
 os.environ.setdefault("NO_CUDA_GRAPH", "1")
 sys.dont_write_bytecode = True
-REF = "/root/reference/MLLM_v2"
+REF = ""          # set by main() from the command line
 
 import numpy as np
 import torch
 
 from . import lm_oracle as L
-from .gen_golden import weights_digest
+from .gen_golden import GOLDEN_THREADS, weights_digest
 
 GOLDEN = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+LOGIT_SAMPLE = 128     # vocabulary columns kept of a tolerance-compared logit tensor
+
+
+def f32_sha256(t: torch.Tensor) -> str:
+    """Digest of the float32 bytes (C order): equal digests <=> bit-equal tensors."""
+    return hashlib.sha256(t.float().contiguous().numpy().tobytes()).hexdigest()
+
+
+def bf16_bits(t: torch.Tensor) -> np.ndarray:
+    """bf16 values as int16 bit patterns; torch.from_numpy(a).view(torch.bfloat16) restores them exactly."""
+    return t.to(torch.bfloat16).contiguous().view(torch.int16).numpy()
+
+
+def sample_cols(n: int) -> torch.Tensor:
+    return torch.randperm(n, generator=torch.Generator().manual_seed(0))[:LOGIT_SAMPLE].sort().values
 
 
 def reference_frames(w, cfg, seqs, dtype):
@@ -140,8 +162,9 @@ def gen_variant(save):
                     assert torch.equal(a, b), f"oracle != reference (gqa): {tag} frame {f} {name}"
         print(f"gqa/partial-rope {tag}: oracle == reference on {frames} streaming frames")
         keep = (0, 1, 15, 16, 19)
-        save[f"gqa_{tag}_out"] = torch.stack([ref[f][0].float() for f in keep]).numpy()
-        save[f"gqa_{tag}_audio_logits"] = torch.stack([ref[f][2].float() for f in keep]).numpy()
+        if tag == "bf16":     # the fp32 run's streaming outputs are checked through its tokens only
+            save["gqa_bf16_out"] = torch.stack([ref[f][0].float() for f in keep]).numpy()
+            save["gqa_bf16_audio_logits_bits"] = bf16_bits(torch.stack([ref[f][2] for f in keep]))
         save[f"gqa_{tag}_tokens"] = torch.stack([ref[f][3] for f in range(frames)]).numpy()
         save["gqa_keep"] = np.array(keep)
         # non-streaming forms on the first T frames (T < context: equal to T streaming steps up to rounding)
@@ -164,8 +187,12 @@ def gen_variant(save):
             assert d <= (2e-6 if dtype == torch.float32 else 4e-2) * max(1.0, r_loc.float().abs().max().item()), (tag, d)
         print(f"gqa/partial-rope {tag}: oracle forward_global_full == reference; forward_local max |diff| {d:.2e} (T={T})")
         save[f"gqa_{tag}_full_out"] = r_out.float().numpy()
-        save[f"gqa_{tag}_full_text_top"] = r_tl.float().topk(8, dim=-1).values.numpy()
-        save[f"gqa_{tag}_local_logits"] = r_loc.float().numpy()
+        if tag == "bf16":
+            save["gqa_bf16_full_text_top"] = r_tl.float().topk(8, dim=-1).values.numpy()
+            save["gqa_bf16_local_argmax"] = r_loc.float().argmax(-1).numpy()
+        cols = sample_cols(r_loc.shape[-1])
+        save["gqa_local_logits_cols"] = cols.numpy()
+        save[f"gqa_{tag}_local_logits_sampled"] = r_loc.float()[..., cols].numpy()
         save[f"gqa_{tag}_local_tokens"] = toks.numpy()
     save["gqa_weights_sha256"] = np.array(weights_digest(L.synthetic_weights(cfg, seed=17, dtype=torch.float32, std=0.05)))
 
@@ -192,14 +219,22 @@ def gen_lora(save):
              "transformer.h.0.mlp.proj.linear.weight"]
     for i, n in enumerate(names):
         assert not torch.equal(msd[n], w[n])
-        save[f"lora_merged_{i}"] = msd[n].numpy()
+        u, s, v = torch.linalg.svd((msd[n].double() - w[n].double()), full_matrices=False)
+        r = int((s > 1e-6 * s[0]).sum())
+        u, v = (u[:, :r] * s[:r]).float(), v[:r].float()
+        assert (w[n] + u @ v - msd[n]).abs().max().item() <= 1e-7, n       # the tests compare to 2e-6
+        save[f"lora_update_{i}_u"], save[f"lora_update_{i}_v"] = u.numpy(), v.numpy()
     save["lora_names"] = np.array(names)
     save["lora_head_rows"] = msd["lm_head.linear.weight"][:64].numpy()
     print("lora: merged weights stored")
 
 
 def main():
-    torch.set_num_threads(min(8, os.cpu_count() or 1))
+    global REF
+    if len(sys.argv) != 2 or not os.path.isdir(os.path.join(sys.argv[1], "models")):
+        sys.exit("usage: python -m oracle.gen_golden_lm <MLLM_v2 directory of the original RSTnet checkout>")
+    REF = os.path.abspath(sys.argv[1])
+    torch.set_num_threads(GOLDEN_THREADS)
     os.makedirs(GOLDEN, exist_ok=True)
     extra = {}
     gen_infer(extra)
@@ -235,7 +270,9 @@ def main():
         keep = (0, 1, 3, 15, 16, 19)
         save[f"{tag}_out"] = torch.stack([ref[f][0].float() for f in keep]).numpy()
         save[f"{tag}_text_top"] = torch.stack([ref[f][1].float().topk(8, dim=-1).values for f in keep]).numpy()
-        save[f"{tag}_audio_logits"] = torch.stack([ref[f][2].float() for f in keep]).numpy()
+        save[f"{tag}_audio_logits_sha256"] = np.array([f32_sha256(ref[f][2]) for f in keep])
+        if tag == "bf16":
+            save["bf16_audio_logits_bits"] = bf16_bits(torch.stack([ref[f][2] for f in keep]))
         save[f"{tag}_tokens"] = torch.stack([ref[f][3] for f in range(frames)]).numpy()
         save[f"{tag}_keep"] = np.array(keep)
         if tag == "f32":

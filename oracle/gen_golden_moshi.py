@@ -17,13 +17,13 @@ import numpy as np
 import torch
 
 from . import moshi_oracle as M
-from .gen_golden import weights_digest
+from .gen_golden import GOLDEN_THREADS, weights_digest
 
 GOLDEN = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
 
 
 def main():
-    torch.set_num_threads(min(8, os.cpu_count() or 1))
+    torch.set_num_threads(GOLDEN_THREADS)
     sys.path.insert(0, REF)
     from models.model import LMGen, LMModel
     cfg = M.SMALL

@@ -240,7 +240,7 @@ def test_streaming_decode_vs_reference_golden(golden_dir, small_lm, graphs):
             n_tok += ref_tokens.numel()
             if f in keep:
                 i = keep.index(f)
-                ro, ra = torch.from_numpy(gold["bf16_out"][i]), torch.from_numpy(gold["bf16_audio_logits"][i])
+                ro, ra = torch.from_numpy(gold["bf16_out"][i]), torch.from_numpy(gold["bf16_audio_logits_bits"][i]).view(BF).float()
                 assert _cos(out, ro) >= 0.999 and _cos(al, ra) >= 0.999, (f, _cos(out, ro), _cos(al, ra))
                 # our deviation from the fp32 evaluation must be of the same size as the reference's own bf16 deviation
                 e_mine, e_ref = _rel(out, t_out), _rel(ro, t_out)
@@ -300,7 +300,7 @@ def _replay_ok(frames, seq, w, cfg, use_sampling, tol):
 def test_inference_imp_vs_reference_loop(golden_dir, small_lm, mode, use_sampling, tk):
     """InferenceImp (infer_no_streaming.py:169-308) as a streaming loop (prefill + forward_step) against the UNMODIFIED
     reference's O(T^2) loop: the reference's bf16 tokens (tests/golden/lm_round2.npz, generated by
-    oracle/gen_golden_lm.py from /root/reference) must be reproduced up to the first bf16 near-tie, and every decision of
+    oracle/gen_golden_lm.py from the original project) must be reproduced up to the first bf16 near-tie, and every decision of
     our own closed loop must be (near-)optimal under the oracle restatement of that loop (pinned bit for bit to the
     reference), which also checks the 2048 / 2049 candidate rules, the delay bookkeeping and the prompt handling."""
     from rstnet_b200.infer import InferenceImp, reverse_delay
@@ -406,7 +406,8 @@ def test_gqa_partial_rope_streaming_vs_reference_golden(gqa_lm):
             tok_ok += int((mine == ref_tokens[f]).sum()); n_tok += mine.numel()
             if f in keep:
                 i = keep.index(f)
-                ro, ra = torch.from_numpy(gold["gqa_bf16_out"][i]), torch.from_numpy(gold["gqa_bf16_audio_logits"][i])
+                ro = torch.from_numpy(gold["gqa_bf16_out"][i])
+                ra = torch.from_numpy(gold["gqa_bf16_audio_logits_bits"][i]).view(BF).float()
                 assert _cos(out, ro) >= 0.999 and _cos(al, ra) >= 0.999, (f, _cos(out, ro), _cos(al, ra))
                 assert _rel(out, ro) <= 5e-2 and _rel(al, ra) <= 5e-2
     print(f"gqa greedy token agreement with the reference: {tok_ok}/{n_tok}")
@@ -467,10 +468,12 @@ def test_forward_local_vs_reference_golden(gqa_lm):
     t_out = torch.from_numpy(gold["gqa_bf16_full_out"]).to(DEV, BF)
     start = m.codecformer_text_emb(toks[:, 0, :])
     lg = m.forward_local(local_start_token=start, sequence=toks[:, 1:, :], transformer_out=t_out)
-    ref = torch.from_numpy(gold["gqa_bf16_local_logits"])
-    assert lg.shape == ref.shape
-    assert _cos(lg, ref) >= 0.999 and _rel(lg, ref) <= 5e-2, (_cos(lg, ref), _rel(lg, ref))
-    agree = float((lg.float().argmax(-1).cpu() == ref.argmax(-1)).float().mean())
+    ref_argmax = torch.from_numpy(gold["gqa_bf16_local_argmax"])                # over the whole vocabulary
+    assert lg.shape[:-1] == ref_argmax.shape and lg.shape[-1] == cfg.audio_card
+    ref = torch.from_numpy(gold["gqa_bf16_local_logits_sampled"])               # a fixed sample of the vocabulary
+    got = lg[..., torch.from_numpy(gold["gqa_local_logits_cols"]).to(DEV)]
+    assert _cos(got, ref) >= 0.999 and _rel(got, ref) <= 5e-2, (_cos(got, ref), _rel(got, ref))
+    agree = float((lg.float().argmax(-1).cpu() == ref_argmax).float().mean())
     print(f"forward_local argmax agreement with the reference: {agree:.3f}")
     assert agree >= 0.9
 

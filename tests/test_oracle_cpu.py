@@ -14,6 +14,16 @@ from oracle import mimi_spec as S
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
+@pytest.fixture(autouse=True)
+def golden_threads():
+    """Run the oracle with the thread count the fixtures were made with: its float32 convolutions round by it."""
+    from oracle.gen_golden import GOLDEN_THREADS
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(n)
+
+
 def test_oracle_cfg1_matches_reference_golden(golden_dir, official_weights):
     g = np.load(os.path.join(golden_dir, "mimi_cfg1.npz"))
     x = S.synthetic_audio(1, 24000, seed=int(g["audio_seed"]))

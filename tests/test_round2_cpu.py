@@ -39,7 +39,8 @@ def test_lora_factors_are_merged_on_load_like_merge_lora_weights(gold):
     sd = m.state_dict()
     assert not any("lora_" in k for k in sd)
     for i, name in enumerate(gold["lora_names"]):
-        ref = torch.from_numpy(gold[f"lora_merged_{i}"])
+        # the reference's merged weight = base + its stored rank-r update (reconstructed to 1e-7)
+        ref = w[str(name)] + torch.from_numpy(gold[f"lora_update_{i}_u"]) @ torch.from_numpy(gold[f"lora_update_{i}_v"])
         assert not torch.equal(sd[str(name)], w[str(name)])
         assert (sd[str(name)] - ref).abs().max().item() <= 2e-6, name
     assert (sd["lm_head.linear.weight"][:64] - torch.from_numpy(gold["lora_head_rows"])).abs().max().item() <= 2e-6
@@ -98,7 +99,8 @@ def test_gqa_partial_rope_oracle_reproduces_reference(gold):
         toks = torch.from_numpy(gold["gqa_f32_local_tokens"])
         loc = L.forward_local(w, cfg, L.scaled_embedding(toks[:, 0, :], w["codecformer_text_emb.weight"]), toks[:, 1:, :],
                               torch.from_numpy(gold["gqa_f32_full_out"]))
-        assert (loc - torch.from_numpy(gold["gqa_f32_local_logits"])).abs().max().item() <= 1e-4
+        cols = torch.from_numpy(gold["gqa_local_logits_cols"])      # fixed sample of the vocabulary
+        assert (loc[..., cols] - torch.from_numpy(gold["gqa_f32_local_logits_sampled"])).abs().max().item() <= 1e-4
     assert agree >= 0.95 * total
 
 
